@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — one "step" = one frame of the hot path (prepass rays + light passes + denoise + tone mapping).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cornell_1080p] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cornell_1080p] [--impl ours|reference] [--dump-outputs DIR]
 
 N = 1: the workload is BASELINE.json configs[1] — cornell 1920x1080, 2 bounces, ReSTIR temporal + spatial (emissive
 and indirect), denoise on — unless --config says otherwise.  N > 1 (launched by torchrun, one rank per GPU): the frame is
@@ -541,6 +541,8 @@ def run_ours(args):
     if rank == 0:
         sampler.stop()
     clocks = sampler.window(t_load_begin, t_load_end) if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dev.readback(L.OUT_TONE_MAPPED))     # frame W + K, the last of both timed arms
 
     # ------------------------------------------------ N > 1: is the frame the ranks assembled the frame one GPU renders?
     # Outside every timed region.  Frames 1..3 from zeroed state through the same tiles + frame assembly as the timed loop; rank 0
@@ -703,6 +705,25 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT = 64_000_000    # bytes --dump-outputs may write, .npy header included
+NPY_HEADER = 4096          # room kept for the header np.save writes (128 bytes for these arrays)
+
+
+def dump_outputs(directory, tone_mapped):
+    """--dump-outputs: the tone-mapped image of the last timed step (what render_frame / run_frame hand a caller), as float32
+    DIR/tone_mapped.npy (H x W x 4).  An image that does not fit DUMP_LIMIT is replaced by a fixed sample of its pixels (seed 0, sorted
+    pixel order): DIR/tone_mapped_sample.npy (n x 4)."""
+    img = np.asarray(tone_mapped, np.float32)
+    name = "tone_mapped"
+    budget = DUMP_LIMIT - NPY_HEADER
+    if img.nbytes > budget:
+        px = img.reshape(-1, img.shape[-1])
+        keep = np.sort(np.random.default_rng(0).choice(px.shape[0], budget // px[0].nbytes, replace=False))
+        img, name = px[keep], "tone_mapped_sample"
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name + ".npy"), img)
+
+
 # ============================================================================================ CPU arms
 def stored_frame_hash(config, frames):
     """sha256 of the tone-mapped frame `frames` of `config` rendered unsharded on one GPU with the default build, committed by
@@ -844,6 +865,9 @@ def run_reference(args):
         st = orc.stats()
         rays += st.tlas_rays + st.blas_rays
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        from bevy_hikari_b200 import layout as L
+        dump_outputs(args.dump_outputs, orc.readback(L.OUT_TONE_MAPPED))
     value = rays / dt / 1e6
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
     full = div == 1
@@ -885,7 +909,14 @@ def main():
     ap.add_argument("--lib", default=None, help="tuning: load this build of libhikari_b200.so (tools/build_variants.py) instead of the in-tree one")
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="N > 1: peer = tiles stored straight into rank 0's frame over NVLink (CUDA IPC); nccl = all_gather of tiles")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the tone-mapped image of the last timed step to DIR as float32 .npy (at most 64 MB: a fixed sample of "
+                         "the pixels of larger images); --gpus 1 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus > 1:
+        ap.error("--dump-outputs: --gpus 1 only")
     args.warmup = max(args.warmup, 3)
     if args.lib:
         from bevy_hikari_b200 import _ffi

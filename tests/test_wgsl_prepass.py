@@ -11,8 +11,9 @@ for three sequences is committed (tests/golden/wgsl_prepass_*.npz, tools/make_wg
     pixel's own footprint, NDC depth to 1e-3 relative, the packed normal to 1 snorm8 step, the depth gradient to 2 %, screen-space
     velocity to 5e-6 + 3e-4 of its magnitude and texture coordinates to 2e-3 — on all but the <= 2 % of pixels where the two methods hit different triangles of
     one instance (an edge inside a mesh, coplanar faces) or where a ground plane recedes to the horizon;
-  * in the build container the fixtures are regenerated from the shader text and must be identical, and four more scenes are rasterised
-    live (a quad through the near plane, the sampler scene, examples/scene.rs with 120 k triangles, the city at twice the size);
+  * in the build container the fixtures are regenerated from the shader text and must be identical;
+  * four more scenes (a quad through the near plane, the sampler scene, examples/scene.rs with 120 k triangles, the city at twice the
+    size) against a window of what the rasteriser made of them (tests/golden/wgsl_prepass_<case>.npz, same tool);
   * `-m gpu`: the CUDA path's G-buffer against the same fixtures with the same bounds (tests/test_gpu_wgsl_golden.py)."""
 import os
 import sys
@@ -104,24 +105,26 @@ def test_oracle_gbuffer_agrees_with_the_rasterised_prepass(case):
 
 
 @pytest.mark.skipif(not IN_CONTAINER, reason="the reference's shader sources exist only in the build container")
-@pytest.mark.parametrize("case", FIXTURE_CASES)
+@pytest.mark.parametrize("case", sorted(WC.PREPASS_CASES))
 def test_committed_prepass_fixtures_are_what_the_shader_text_rasterises_today(case):
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     sys.path.insert(0, os.path.join(ROOT, "oracle", "wgsl"))
     import make_wgsl_golden
-    r = make_wgsl_golden.run_prepass_case(case)
-    want = fixture(case)
+    r = make_wgsl_golden.prepass_fixture(case)
+    z = np.load(os.path.join(GOLDEN, f"wgsl_prepass_{case}.npz"))
     for k, _ in WC.PREPASS_PLANES:
-        assert np.array_equal(np.ascontiguousarray(r[k]).view(np.uint8), np.ascontiguousarray(want[k]).view(np.uint8)), (case, k)
+        assert np.array_equal(np.ascontiguousarray(r[k]).view(np.uint8), np.ascontiguousarray(z[k]).view(np.uint8)), (case, k)
+    if "skipped_triangles" in z:
+        assert int(r["skipped_triangles"]) == int(z["skipped_triangles"])
 
 
-@pytest.mark.skipif(not IN_CONTAINER, reason="the reference's shader sources exist only in the build container")
-@pytest.mark.parametrize("case", sorted(c for c, v in WC.PREPASS_CASES.items() if not v[7]))
-def test_more_scenes_rasterised_live(case):
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    sys.path.insert(0, os.path.join(ROOT, "oracle", "wgsl"))
-    import make_wgsl_golden
-    raster = make_wgsl_golden.run_prepass_case(case)
-    assert raster["skipped_triangles"] == 0 or case == "town"      # degenerate clipped slivers only
+@pytest.mark.parametrize("case", sorted(WC.PREPASS_WINDOWS))
+def test_more_scenes_against_a_window_of_the_rasterised_prepass(case):
+    """what the rasteriser made of these scenes is stored for a window of the frame (WC.PREPASS_WINDOWS); the oracle's G-buffer is
+    compared on the same window"""
+    z = np.load(os.path.join(GOLDEN, f"wgsl_prepass_{case}.npz"))
+    assert int(z["skipped_triangles"]) == 0 or case == "town"      # degenerate clipped slivers only
     bench, g = render_gbuffer(case, lambda b: b.oracle(), lambda r, b: r.update_instances_desc(b.world.scene_desc()))
-    compare(raster, g, bench.width, bench.height, case)
+    x0, x1, y0, y1 = WC.PREPASS_WINDOWS[case]
+    compare({k: z[k] for k, _ in WC.PREPASS_PLANES}, {which: WC.prepass_window(case, a, bench.width, bench.height) for which, a in g.items()},
+            x1 - x0, y1 - y0, case)

@@ -80,6 +80,34 @@ def digest(array):
     return hashlib.sha256(np.ascontiguousarray(array).tobytes()).hexdigest()
 
 
+def load_digests(path):
+    """{name: hex digest} of a digest fixture (tools/make_wgsl_golden.py: `names` + raw SHA-256 `digests`)"""
+    z = np.load(path)
+    return {str(n): bytes(d).hex() for n, d in zip(z["names"], z["digests"])}
+
+
+def save_digests(path, digests, **extra):
+    names = sorted(digests)
+    np.savez_compressed(path, names=np.array(names), digests=np.array([np.frombuffer(bytes.fromhex(digests[n]), np.uint8) for n in names]),
+                        **extra)
+
+
+# ------------------------------------------------------------------------------------------------ pass by pass
+# Every pass of the reference's shader text run FROM THE ORACLE'S STATE (before each pass the reference's planes are overwritten with the
+# oracle's): scene, config, size; PER_PASS_FRAMES frames, the camera translating by PER_PASS_STEP per frame.  The digest of every plane
+# after every pass is stored in tests/golden/wgsl_per_pass_<scene>.npz (a per-pass diagnosis of any drift).
+PER_PASS_CASES = [("cornell", "cornell_1080p", (48, 40)), ("city", "city_4k", (64, 36)), ("simple", "city_8k", (48, 32))]
+PER_PASS_FRAMES, PER_PASS_STEP = 6, (0.02, 0.0, -0.01)
+PASS_PLANES = PLANES[:-1]          # albedo, render and variance of the three signals, the ten reservoir buffers
+
+
+def light_passes(inp):
+    """the passes of LightNode::run in order; the spatial reuses when the frame enables them"""
+    from oracle import oracle as O
+    return ([O.PASS_ALBEDO, O.PASS_DIRECT, O.PASS_EMISSIVE] + ([O.PASS_EMISSIVE_SPATIAL] if inp.frame.emissive_spatial_reuse else []) +
+            [O.PASS_INDIRECT] + ([O.PASS_INDIRECT_SPATIAL] if inp.frame.indirect_spatial_reuse else []))
+
+
 def make_bench(case):
     from tests.conftest import Bench
     scene, config, (w, h), frames, step, animation, overrides = CASES[case]
@@ -141,8 +169,22 @@ PREPASS_CASES = {
     "town": ("town", "scene_1080p", (128, 72), 1, (0.0, 0.0, 0.0), None, False, False),                       # examples/scene.rs, 120 k triangles
     "city_larger": ("city", "city_4k", (256, 144), 2, (0.05, 0.0, -0.04), None, False, False),
 }
+# the cases without a committed full-frame fixture: their fixtures hold this window (x0, x1, y0, y1) of the compared frame, which keeps
+# each file small.  The oracle against the rasterised G-buffer, full frame -> window (tools/make_wgsl_golden.py --prepass prints both):
+#   simple_ground_plane  covered pixels 4550 -> 1442; beyond a bound: position 76 -> 15, depth 17 -> 4, gradient 1 -> 1
+#   samplers             the whole frame (3630 covered, none beyond any bound)
+#   town                 covered 8903 -> 2304; id mismatches 6 -> 2, normal 14 -> 5, gradient 27 -> 8; position 136, depth 54, uv 3 -> 0
+#   city_larger          covered 26177 -> 2223; id mismatches 1 -> 1, gradient 40 -> 8; normal 15, position 3, depth 2, velocity 2, uv 2 -> 0
+PREPASS_WINDOWS = {"simple_ground_plane": (24, 72, 16, 48), "samplers": (0, 96, 0, 64), "town": (32, 96, 18, 54),
+                   "city_larger": (96, 160, 54, 90)}
 PREPASS_PLANES = [("position", L.OUT_GBUFFER_POSITION), ("normal", L.OUT_GBUFFER_NORMAL), ("depth_gradient", L.OUT_GBUFFER_DEPTH_GRADIENT),
                   ("instance_material", L.OUT_GBUFFER_INSTANCE_MATERIAL), ("velocity_uv", L.OUT_GBUFFER_VELOCITY_UV)]
+
+
+def prepass_window(case, plane, width, height):
+    """`plane` (a full frame of `case`) cut to the case's PREPASS_WINDOWS entry"""
+    x0, x1, y0, y1 = PREPASS_WINDOWS[case]
+    return np.ascontiguousarray(np.ascontiguousarray(plane).reshape(height, width, -1)[y0:y1, x0:x1])
 
 
 def prepass_sequence(case):

@@ -3,7 +3,8 @@
 instance animation; every frame is computed twice — by the reference's own shader text (oracle/wgsl/: light / denoise / tone mapping /
 SMAA / TAA WGSL and the FSR 1.0 GLSL, translated and executed with the wiring of light.rs / post_process.rs) and by the CPU oracle — and
 every buffer and texture of every frame must be identical, bit for bit.  The committed fixtures (tests/golden/wgsl_*.npz) are 23 chosen
-sequences; this walks the space between them.
+sequences; this walks the space between them.  The reference's planes of FIXED_SEEDS are committed too (tests/golden/wgsl_pin_seeds.npz),
+so tests/test_wgsl_reference.py runs the oracle side of those (oracle_digests) anywhere.
 
 usage: tools/fuzz_wgsl_pin.py FIRST_SEED COUNT
 
@@ -22,8 +23,6 @@ from bevy_hikari_b200 import layout as L  # noqa: E402
 from bevy_hikari_b200 import plugin  # noqa: E402
 from tests import wgsl_cases as WC  # noqa: E402
 from tests.conftest import Bench, cornell_animation  # noqa: E402
-import make_wgsl_golden as G  # noqa: E402
-import run_reference as R  # noqa: E402
 
 SCENES = [("cornell", "cornell_1080p"), ("cornell", "cornell_256"), ("simple", "cornell_1080p"), ("samplers", "cornell_1080p"),
           ("city", "city_4k"), ("city", "city_8k"), ("minimal", "cornell_1080p")]
@@ -53,50 +52,90 @@ def random_case(rng):
     return scene, config, (w, h), settings, upscalers, step, animated, frames
 
 
-def run(seed):
-    rng = np.random.default_rng(seed)
-    scene, config, (w, h), settings, upscalers, step, animated, frames = random_case(rng)
-    bench = Bench(scene, w, h, config=config, **settings)
+# the seeds whose reference planes are committed (tests/golden/wgsl_pin_seeds.npz, tools/make_wgsl_golden.py --pin-seeds)
+FIXED_SEEDS = list(range(5000, 5010))
+
+
+class Case:
+    """the random case of `seed`: bench, planes compared, frame inputs"""
+
+    def __init__(self, seed):
+        rng = np.random.default_rng(seed)
+        scene, config, (w, h), settings, self.upscalers, self.step, animated, self.frames = random_case(rng)
+        self.bench = bench = Bench(scene, w, h, config=config, **settings)
+        self.anim = cornell_animation(bench) if animated else None
+        self.smaa = self.upscalers and bench.settings.upscale_kind == plugin.UPSCALE_SMAA_TU4X
+        self.taa = self.upscalers and bench.settings.taa == plugin.TAA_JASMINE
+        self.fsr = self.upscalers and bench.settings.upscale_kind == plugin.UPSCALE_FSR1
+        planes = list(WC.PLANES) + (WC.DENOISED[:3 if bench.settings.indirect_bounces else 2] if bench.settings.denoise else [])
+        planes += ([("upscaled", L.OUT_UPSCALED)] if self.smaa else []) + ([("taa", L.OUT_TAA)] if self.taa else [])
+        planes += [("fsr_easu", L.OUT_UPSCALED), ("fsr_rcas", L.OUT_FSR_SHARPENED)] if self.fsr else []
+        self.planes = planes
+        self.what = (f"{scene}/{config} {w}x{h} {self.frames} frames upscalers={self.upscalers} step={tuple(round(s, 3) for s in self.step)} "
+                     f"animated={animated} {settings}")
+
+    def inputs(self, f):
+        inp = self.bench.moving_inputs(f, self.step) if any(self.step) else self.bench.inputs(f)
+        if self.upscalers:
+            inp.temporal_upscalers = 1
+        return inp
+
+
+def reference_digests(seed):
+    """{f<frame>_<plane>: digest} of every plane of every frame as the reference's shader text computes them (G-buffer: the oracle's)"""
+    import make_wgsl_golden as G
+    import run_reference as R
+    c = Case(seed)
+    bench = c.bench
+    w, h = bench.width, bench.height
     textures = [(np.ascontiguousarray(t["rgba"]), t["address_mode_u"], t["address_mode_v"], t["filter_linear"], t["srgb"]) for t in bench.scene.textures]
     ref = R.WgslReference(bench.world.buffers(), textures, plugin.load_noise(), w, h, bench.settings.upscale_ratio)
-    orc_g, orc = bench.oracle(), bench.oracle()
-    anim = cornell_animation(bench) if animated else None
-    smaa = upscalers and bench.settings.upscale_kind == plugin.UPSCALE_SMAA_TU4X
-    taa = upscalers and bench.settings.taa == plugin.TAA_JASMINE
-    fsr = upscalers and bench.settings.upscale_kind == plugin.UPSCALE_FSR1
-    planes = list(WC.PLANES) + (WC.DENOISED[:3 if bench.settings.indirect_bounces else 2] if bench.settings.denoise else [])
-    planes += ([("upscaled", L.OUT_UPSCALED)] if smaa else []) + ([("taa", L.OUT_TAA)] if taa else [])
-    planes += [("fsr_easu", L.OUT_UPSCALED), ("fsr_rcas", L.OUT_FSR_SHARPENED)] if fsr else []
-    bad = []
-    for f in range(1, frames + 1):
-        if anim:
-            anim.step(f)
-            for o in (orc, orc_g):
-                o.update_instances_desc(bench.world.scene_desc())
+    orc_g = bench.oracle()
+    out = {}
+    for f in range(1, c.frames + 1):
+        if c.anim:
+            c.anim.step(f)
+            orc_g.update_instances_desc(bench.world.scene_desc())
             ref.scene = {k: np.ascontiguousarray(v) for k, v in bench.world.buffers().items()}
-        inp = bench.moving_inputs(f, step) if any(step) else bench.inputs(f)
-        if upscalers:
-            inp.temporal_upscalers = 1
+        inp = c.inputs(f)
         orc_g.prepass(inp)
         ref.set_gbuffer(*[np.ascontiguousarray(orc_g.readback(k)) for k in WC.GBUFFER])
         ref.light_node(inp)
         ref.post_process_node(inp, bool(bench.settings.denoise))
-        if smaa or taa:
-            ref.upscale_node(inp, smaa, taa)
-        if fsr:
-            ref.fsr_node(inp, taa, bench.settings.upscale_sharpness)
-        orc.render_frame(inp)
+        if c.smaa or c.taa:
+            ref.upscale_node(inp, c.smaa, c.taa)
+        if c.fsr:
+            ref.fsr_node(inp, c.taa, bench.settings.upscale_sharpness)
         got = G.reference_planes(ref, bench)
-        for name, which in planes:
-            a = np.ascontiguousarray(got[name]).view(np.uint8).reshape(-1)
-            b = np.ascontiguousarray(orc.readback(which)).view(np.uint8).reshape(-1)
-            if a.size != b.size or not np.array_equal(a, b):
-                bad.append((f, name))
-    what = f"{scene}/{config} {w}x{h} {frames} frames upscalers={upscalers} step={tuple(round(s, 3) for s in step)} animated={animated} {settings}"
+        for name, _ in c.planes:
+            out[f"f{f}_{name}"] = WC.digest(got[name])
+    return out, c.what
+
+
+def oracle_digests(seed):
+    """the same planes as the CPU oracle renders them"""
+    c = Case(seed)
+    orc = c.bench.oracle()
+    out = {}
+    for f in range(1, c.frames + 1):
+        if c.anim:
+            c.anim.step(f)
+            orc.update_instances_desc(c.bench.world.scene_desc())
+        orc.render_frame(c.inputs(f))
+        for name, which in c.planes:
+            out[f"f{f}_{name}"] = WC.digest(orc.readback(which))
+    return out, c.what
+
+
+def run(seed):
+    ref, what = reference_digests(seed)
+    orc, _ = oracle_digests(seed)
+    bad = [k for k in ref if orc[k] != ref[k]]
     return bad, what
 
 
 def main():
+    import run_reference as R
     if not R.available():
         raise SystemExit("needs /root/reference and g++ (build container only)")
     first, count = int(sys.argv[1]), int(sys.argv[2])

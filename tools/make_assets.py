@@ -12,6 +12,7 @@ are committed:
   scenes/town.npz                 <- assets/models/scene.gltf          (examples/scene.rs:80-84; BASELINE configs[2]),
                                      84 meshes / 120 440 triangles / 66 materials; the 52 embedded PNGs are shipped
                                      box-filtered to at most 256 x 256 (--scene)
+  tests/golden/gltf_houses.json   <- the three house GLBs: what rebuilds them from scenes/house*.npz (--house-fixture)
 
 A scene file holds what a Bevy app would hand to the plugin: meshes (position/normal/uv/indices per glTF
 primitive), per-instance (mesh, material, world transform), StandardMaterial parameters, RGBA8 textures.
@@ -136,6 +137,16 @@ def decode_image(js, bufs, image_index, base_dir):
     return np.asarray(im.convert("RGBA"), np.uint8).copy()
 
 
+def box_filtered(img, max_tex):
+    """`img` box-filtered so that its larger side is at most `max_tex` (None: unchanged)"""
+    if max_tex and max(img.shape[:2]) > max_tex:
+        from PIL import Image
+        s = max_tex / max(img.shape[:2])
+        img = np.asarray(Image.fromarray(img).resize((max(1, int(img.shape[1] * s)), max(1, int(img.shape[0] * s))),
+                                                     Image.BOX), np.uint8).copy()
+    return img
+
+
 def convert_gltf(path, max_tex=None):
     """Return dict of arrays: meshes, instances (depth-first node order), materials, textures."""
     js, bufs = load_gltf(path) if path.endswith(".gltf") else load_glb(path)
@@ -217,13 +228,7 @@ def convert_gltf(path, max_tex=None):
     out["tex_count"] = np.array(len(tex_images), np.uint32)
     base_dir = os.path.dirname(path)
     for ti, (src, srgb, sampler) in enumerate(tex_images):
-        img = decode_image(js, bufs, src, base_dir)
-        if max_tex and max(img.shape[:2]) > max_tex:
-            from PIL import Image
-            s = max_tex / max(img.shape[:2])
-            img = np.asarray(Image.fromarray(img).resize((max(1, int(img.shape[1] * s)), max(1, int(img.shape[0] * s))),
-                                                         Image.BOX), np.uint8).copy()
-        out[f"t{ti}_rgba"] = img
+        out[f"t{ti}_rgba"] = box_filtered(decode_image(js, bufs, src, base_dir), max_tex)
         smp = js["samplers"][sampler] if sampler is not None and "samplers" in js else {}
         wrap = {10497: 0, 33071: 1, 33648: 2}
         out[f"t{ti}_info"] = np.array([wrap[smp.get("wrapS", 10497)], wrap[smp.get("wrapT", 10497)],
@@ -245,7 +250,42 @@ def make_noise():
     print("noise", arr.shape, arr.mean())
 
 
+HOUSES = (("house", "Big House.glb"), ("house2", "Big House 2.glb"), ("house3", "Big House 3.glb"))
+
+
+def house_fixture():
+    """tests/golden/gltf_houses.json: what tests/test_gltf_ingest.py needs to rebuild the three house GLBs (5 to 7 MB each, nearly all
+    of it PNG) from the shipped scene files: each file's JSON chunk, the SHA-256 of its geometry bytes (every buffer view that is not an
+    image), and for each image the scene-file texture that holds it box-filtered, with the PNG's colour mode"""
+    import hashlib
+    from PIL import Image
+    out = {}
+    for name, fn in HOUSES:
+        js, bufs = load_glb(f"{REF}/assets/models/Low Poly/{fn}")
+        z = np.load(f"{ROOT}/scenes/{name}.npz")
+        views = js["bufferViews"]
+        image_views = {im["bufferView"] for im in js["images"]}
+        geometry = b"".join(bufs[0][v.get("byteOffset", 0):v.get("byteOffset", 0) + v["byteLength"]]
+                            for i, v in enumerate(views) if i not in image_views)
+        texture, mode = [], []
+        for i, im in enumerate(js["images"]):
+            v = views[im["bufferView"]]
+            m = Image.open(io.BytesIO(bufs[0][v.get("byteOffset", 0):v.get("byteOffset", 0) + v["byteLength"]])).mode
+            assert m in ("RGB", "RGBA"), (fn, i, m)
+            img = box_filtered(decode_image(js, bufs, i, None), 512)
+            texture.append(next(t for t in range(int(z["tex_count"])) if np.array_equal(z[f"t{t}_rgba"], img)))
+            mode.append(m)
+        out[fn] = {"npz": name, "json": js, "geometry_sha256": hashlib.sha256(geometry).hexdigest(), "image_texture": texture,
+                   "image_mode": mode}
+    with open(f"{ROOT}/tests/golden/gltf_houses.json", "w") as f:
+        json.dump(out, f, indent=None, separators=(",", ":"))
+        f.write("\n")
+
+
 def main():
+    if "--house-fixture" in sys.argv:
+        house_fixture()
+        return
     make_noise()
     os.makedirs(f"{ROOT}/scenes", exist_ok=True)
     c = convert_gltf(f"{REF}/assets/models/cornell.glb")
@@ -256,7 +296,7 @@ def main():
         from PIL import Image
         earth = Image.open(f"{REF}/assets/models/Earth/earth_daymap.jpg").convert("RGBA").resize((512, 256), Image.BOX)
         np.savez_compressed(f"{ROOT}/scenes/earth.npz", rgba=np.asarray(earth, np.uint8))
-        for name, fn in (("house", "Big House.glb"), ("house2", "Big House 2.glb"), ("house3", "Big House 3.glb")):
+        for name, fn in HOUSES:
             h = convert_gltf(f"{REF}/assets/models/Low Poly/{fn}", max_tex=512)
             np.savez_compressed(f"{ROOT}/scenes/{name}.npz", **h)
             print(name, "meshes", int(h["mesh_count"]), "instances", len(h["inst_mesh"]), "textures", int(h["tex_count"]),
